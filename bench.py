@@ -3,6 +3,7 @@
 all-reduce for N > 1), images/s, on N B200s of one box (BASELINE.json: metric / configs[1], configs[2]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload unet|ae|clip] [--impl b200|reference|torch_gpu]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -225,7 +226,7 @@ def run_reference(args, rank, world):
     import torch
     cores = os.cpu_count() or 1
     batch = 4  # BASELINE.json configs[0]: the reference's CPU-runnable case; a bounded sample of the per-GPU step
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     warm = 1
     s_per_step = cpu_port_step_time(batch, args.size, steps, warm, cores, args.workload)
     v = batch / s_per_step
@@ -261,7 +262,7 @@ def run_torch_gpu(args, rank, world):
     for _ in range(max(args.warmup, 3)):
         step()
     torch.cuda.synchronize()
-    k = max(1, min(args.steps, 10))
+    k = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(k):
@@ -346,7 +347,35 @@ class Workload:
         else:
             loss = self.loss_fn(out, batch["mask"])
         loss.backward()
+        # detached: no autograd graph of an eager step stays alive into a CUDA-graph capture; under replay these are
+        # the graph's static output buffers
+        self.outputs = (out.detach(), loss.detach())
         return loss
+
+
+def dump_outputs(path, wl):
+    """What the last step of `wl` handed its caller -- loss, model output, every parameter gradient -- as float32
+    DIR/loss.npy, DIR/output.npy and DIR/grad.<parameter name>.npy.  An array larger than its cap is written as a fixed
+    sample: the elements at sorted indices drawn by a generator seeded with 0, the same for every build.  The caps keep
+    the files under 64 MB in all (16 MB of output, at most 40 MB of gradients)."""
+    import numpy as np
+    import torch
+
+    def flat_sample(t, cap):
+        t = t.detach()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        return t.float().cpu().numpy()
+
+    out, loss = wl.outputs
+    grads = [(n, p.grad) for n, p in wl.model.named_parameters() if p.grad is not None]
+    grad_cap = min(1 << 16, (40 << 20) // (4 * len(grads)))
+    arrays = {"loss": flat_sample(loss, 1), "output": flat_sample(out, 1 << 22)}
+    arrays.update(("grad." + n, flat_sample(g, grad_cap)) for n, g in grads)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def main():
@@ -364,7 +393,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="skip the CUDA-graph replay leg")
     ap.add_argument("--clip-dense", action="store_true", help="clip workload: dense per-patch features instead of the "
                     "reference extractor's pooled embedding expanded over the grid")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, model output and parameter gradients of the "
+                    "last timed step to DIR/<name>.npy (float32; large arrays as a fixed sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 step computes; it does not apply to --impl " + args.impl)
     if args.batch <= 0:
         args.batch = WORKLOADS[args.workload][1]
     rank = int(os.environ.get("RANK", "0"))
@@ -481,6 +516,8 @@ def main():
 
         if sampler and attempt == 0:
             sampler.samples.clear()  # keep only what was sampled during the timed regions
+        # every attempt draws the same dropout masks, so the last step's outputs depend on --steps alone
+        torch.manual_seed(99 + rank)
         ms = timed(marked_step, args.steps)
         per_rank_resident = timed.per_rank_ms
         per = sorted(marks[i].elapsed_time(marks[i + 1]) for i in range(args.steps))
@@ -493,6 +530,8 @@ def main():
         remeasured = f"first attempt had a {worst:.1f} ms step against a median of {med:.1f} ms ({ms / args.steps:.2f} ms/step); measured again"
     ms_per_step = ms / args.steps
     value = world * B / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl)
     # the eager form of the same step (also the launch count: a graph replay launches the same kernels as graph nodes)
     l0 = _lib.call("b200unet_launch_count")
     step()

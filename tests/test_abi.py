@@ -3,6 +3,8 @@ _lib.py covers the same set.  No compute entry point is called (there is no GPU 
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -53,16 +55,22 @@ def test_statistics_slots_cover_the_cta_pair_layout():
 
 
 def test_product_path_fails_loudly_without_a_device():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("needs a CPU-only host")
-    from unet_implementations_b200.models.losses import SimpleLoss
-    from unet_implementations_b200.models.unet import UNet
-    m = UNet(n_stages=2, features_per_stage=[32, 32], encoder_dropout_rates=[0, 0], decoder_dropout_rates=[0])
-    with pytest.raises(RuntimeError, match="no CPU path"):
-        m(torch.zeros(1, 3, 16, 16))
-    with pytest.raises(RuntimeError, match="no CPU path"):
-        SimpleLoss()(torch.zeros(1, 3, 8, 8), torch.zeros(1, 8, 8, dtype=torch.long))
+    # a child process with every GPU hidden, so that a GPU host checks the CPU-only case too
+    code = (
+        "import pytest, torch\n"
+        "assert not torch.cuda.is_available()\n"
+        "from unet_implementations_b200.models.losses import SimpleLoss\n"
+        "from unet_implementations_b200.models.unet import UNet\n"
+        "m = UNet(n_stages=2, features_per_stage=[32, 32], encoder_dropout_rates=[0, 0], decoder_dropout_rates=[0])\n"
+        "with pytest.raises(RuntimeError, match='no CPU path'):\n"
+        "    m(torch.zeros(1, 3, 16, 16))\n"
+        "with pytest.raises(RuntimeError, match='no CPU path'):\n"
+        "    SimpleLoss()(torch.zeros(1, 3, 8, 8), torch.zeros(1, 8, 8, dtype=torch.long))\n"
+        "print('ok')\n"
+    )
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=ROOT, timeout=300)
+    assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout[-2000:] + r.stderr[-4000:]
 
 
 def test_missing_library_is_an_error(monkeypatch, tmp_path):

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 from conftest import ROOT
 
 
@@ -31,3 +34,25 @@ def test_other_ranks_of_the_reference_arm_exit_quietly():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                         "--size", "64"], capture_output=True, text=True, timeout=300, cwd=ROOT, env=env)
     assert r.returncode == 0 and not [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_from_run_to_run(tmp_path):
+    """--dump-outputs writes the loss, model output and every parameter gradient of the last timed step as float32
+    .npy files, at most 64 MB in all, and two runs with the same arguments write the same arrays."""
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--batch", "2",
+                            "--size", "64", "--no-cpu-baseline", "--no-profile", "--no-e2e", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert len([ln for ln in r.stdout.splitlines() if ln.startswith("{")]) == 1
+        dumps.append({f: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = dumps
+    assert len(a) == 2 + 90 and a["loss.npy"].shape == () and a["output.npy"].shape == (2, 3, 64, 64)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert a.keys() == b.keys()
+    for k in a:
+        assert a[k].dtype == np.float32 and np.isfinite(a[k]).all(), k
+        assert np.array_equal(a[k], b[k]), k
