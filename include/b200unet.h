@@ -354,6 +354,20 @@ int b200unet_sgd_flat_step(const b200unet_flat_tensor* table_dev, int count, int
                            const float* grad, float* momentum_buf, float lr, float momentum, float weight_decay,
                            int nesterov, float grad_scale, const float* lr_dev /* device scalar overriding lr, or NULL */,
                            void* stream);
+/* adam_flat_step -- torch.optim.Adam(lr, betas, eps, weight_decay, decoupled_weight_decay) (AdamW when decoupled != 0),
+ *   the optimizer of the autoencoder's trainer (AE_pretrained/reconstruction/src/train.py:390-394), over the same flat
+ *   buffers and descriptor table as sgd_flat_step, packs included: master / gradient / exp_avg / exp_avg_sq at the
+ *   same element offsets.  The arithmetic is torch 2.11's `_multi_tensor_adam` (torch/optim/adam.py, capturable=False)
+ *   operation by operation: bit-exact with torch.optim.Adam on CUDA for grad_scale 1 (or a power of two).
+ *   steps: DEVICE fp32 [count], the per-tensor step counts (torch's state["step"]), advanced for every tensor whose
+ *   flags bit 0 is set; scalars_ws: DEVICE fp32 [4 * count], 16-byte aligned, scratch for the per-tensor scalars.
+ *   Two launches on `stream` (a one-block prologue that advances the counts and forms the bias corrections in double,
+ *   then the flat step), so that a CUDA graph of the step replays both.  lr_dev: DEVICE fp64 scalar overriding lr,
+ *   or NULL.  Flags bit 1 is ignored: zero moments are Adam's initial state. */
+int b200unet_adam_flat_step(const b200unet_flat_tensor* table_dev, int count, int total_blocks, float* master,
+                            const float* grad, float* exp_avg, float* exp_avg_sq, float* steps, float* scalars_ws,
+                            double lr, const double* lr_dev, double beta1, double beta2, double eps, double weight_decay,
+                            int decoupled, float grad_scale, void* stream);
 int b200unet_argmax_counts(const float* logits_nchw, const int64_t* target, int ignore_index, int64_t* pred_or_null,
                            int64_t* counts9, int N, int64_t HW, void* stream);
 

@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int64, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_float, c_int, c_int64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B200UNET_LIB") or os.path.join(_HERE, "libb200unet.so")  # env: developer A/B of two builds
@@ -58,7 +58,7 @@ class FlatTensor(Structure):
     ]
 
 
-_P, _I, _L, _F = c_void_p, c_int, c_int64, c_float
+_P, _I, _L, _F, _D = c_void_p, c_int, c_int64, c_float, c_double
 
 # name -> (restype, argtypes); restype c_int means "status code, raise on non-zero"
 SIGNATURES = {
@@ -131,6 +131,7 @@ SIGNATURES = {
     "b200unet_sgd_flat_step": (c_int, [_P, _I, _I, _P, _P, _P, _F, _F, _F, _I, _F, _P, _P]),
     "b200unet_sgd_max_tensors": (c_int, []),
     "b200unet_sgd_nesterov_step": (c_int, [_P, _P, _P, _P, _I, _F, _F, _F, _I, _I, _P]),
+    "b200unet_adam_flat_step": (c_int, [_P, _I, _I, _P, _P, _P, _P, _P, _P, _D, _P, _D, _D, _D, _D, _I, _F, _P]),
     "b200unet_argmax_counts": (c_int, [_P, _P, _I, _P, _P, _I, _L, _P]),
     "b200unet_recon_head_fwd": (c_int, [_P, _L, _P, _P, _I, _L, _I, _P]),
     "b200unet_recon_head_fwd_f32": (c_int, [_P, _L, _P, _P, _I, _L, _I, _P]),

@@ -1,6 +1,8 @@
 // The two steps either side of the hot path in the reference's trainer (SURVEY.md section 8f):
 //  * the optimizer step -- torch.optim.SGD(momentum, nesterov=True, weight_decay) over the model's 90 parameter
-//    tensors (Our_UNet/src/train.py:431-451) as ONE multi-tensor launch instead of ~5 foreach launches per step;
+//    tensors (Our_UNet/src/train.py:431-451) as ONE multi-tensor launch instead of ~5 foreach launches per step, and
+//    torch.optim.Adam / AdamW (the autoencoder's, AE_pretrained/reconstruction/src/train.py:390-394) over the flat
+//    buffers;
 //  * the validation metric -- argmax over the 3 logits + per-class intersection / prediction / target counts over
 //    the valid pixels (train.py:554-572, nine .item() host syncs per batch in the reference) as one pass with integer
 //    counters (bit-exact) and no host sync.
@@ -57,25 +59,124 @@ __global__ void __launch_bounds__(kSgdThreads) sgd_nesterov_kernel(const __grid_
 }
 
 // ------------------------------------------------------------------------------------------------ flat optimizer step
-// SURVEY.md 8f row 1 as written: ONE launch over the flat fp32 master / gradient / momentum buffers that (i) applies
-// the all-reduce epilogue scale to the gradient, (ii) does the SGD-Nesterov update of sgd_nesterov_kernel (same
-// operations in the same order: bit-exact with torch.optim.SGD for scale 1) and (iii) emits the bf16 operand packs
-// the conv kernels consume -- [Cout][3][3][Cin] (fprop), [Cin][3][3][Cout] (dgrad) and the parity-stacked stride-2
-// dgrad pack -- so that no repack kernel runs between the optimizer and the next forward and the packs can never be
-// stale.  The 3x3 weights of the tensor-core layers (99.9 % of the parameters) are processed in 32 x 32 x 9 tiles
-// through shared memory so that the fp32 traffic AND the pack stores are coalesced; every other tensor (norm
-// parameters, biases, the stem, 1x1 and padded heads) is walked element by element in storage order.
+// SURVEY.md 8f row 1 as written: ONE launch over the flat fp32 master / gradient / optimizer-state buffers that (i)
+// applies the all-reduce epilogue scale to the gradient, (ii) updates master + state with an update rule (SgdRule:
+// the SGD-Nesterov update of sgd_nesterov_kernel; AdamRule: torch's foreach Adam / AdamW; both bit-exact with torch
+// for scale 1) and (iii) emits the bf16 operand packs the conv kernels consume -- [Cout][3][3][Cin] (fprop),
+// [Cin][3][3][Cout] (dgrad) and the parity-stacked stride-2 dgrad pack -- so that no repack kernel runs between the
+// optimizer and the next forward and the packs can never be stale.  The 3x3 weights of the tensor-core layers (99.9 %
+// of the parameters) are processed in 32 x 32 x 9 tiles through shared memory so that the fp32 traffic AND the pack
+// stores are coalesced; every other tensor (norm parameters, biases, the stem, 1x1 and padded heads) is walked element
+// by element in storage order.
 constexpr int kFlatThreads = 256, kFlatPerThread = 4;
 
-__global__ void __launch_bounds__(kFlatThreads) sgd_flat_kernel(const b200unet_flat_tensor* __restrict__ T, int count,
-                                                                 float* __restrict__ master,
-                                                                 const float* __restrict__ grad,
-                                                                 float* __restrict__ mom, float lr_arg, float momentum,
-                                                                 float wd, int nesterov, float grad_scale,
-                                                                 const float* __restrict__ lr_dev) {
-  // the learning rate as a device scalar (when given) keeps a CUDA graph of the whole training step valid across
-  // LambdaLR updates (train.py:454-477): the host rewrites one float instead of re-capturing
-  const float lr = lr_dev ? __ldg(lr_dev) : lr_arg;
+// An update rule is built per block from the launch arguments and the block's tensor, and maps an element index of
+// that tensor to its new master value (writing the optimizer state on the way); flat_step_kernel does the rest.
+struct SgdRule {
+  struct Args {
+    float* master;
+    const float* grad;
+    float* mom;
+    float lr, momentum, wd, grad_scale;
+    int nesterov;
+    const float* lr_dev;
+  };
+  float* __restrict__ p;
+  const float* __restrict__ g;
+  float* __restrict__ buf;
+  float lr, momentum, wd, grad_scale;
+  bool nesterov, first;
+  __device__ __forceinline__ SgdRule(const Args& a, int, const b200unet_flat_tensor& D)
+      : p(a.master + D.offset), g(a.grad + D.offset), buf(a.mom ? a.mom + D.offset : nullptr),
+        // the learning rate as a device scalar (when given) keeps a CUDA graph of the whole training step valid across
+        // LambdaLR updates (train.py:454-477): the host rewrites one float instead of re-capturing
+        lr(a.lr_dev ? __ldg(a.lr_dev) : a.lr), momentum(a.momentum), wd(a.wd), grad_scale(a.grad_scale),
+        nesterov(a.nesterov != 0), first((D.flags & 2) != 0) {}
+  // torch's CUDA foreach SGD arithmetic, operation by operation
+  __device__ __forceinline__ float operator()(int i) const {
+    const float pv = p[i];
+    float gv = __ldg(g + i);
+    // every load before the first store: the compiler predicates the momentum path instead of branching around it,
+    // and the loads of consecutive elements overlap
+    const bool has_buf = momentum != 0.f;
+    const float bo = has_buf && !first ? buf[i] : 0.f;
+    if (grad_scale != 1.f) gv = __fmul_rn(gv, grad_scale);
+    if (wd != 0.f) gv = fmaf(wd, pv, gv);
+    float upd = gv;
+    if (has_buf) {
+      const float bv = first ? gv : __fadd_rn(__fmul_rn(bo, momentum), gv);
+      buf[i] = bv;
+      upd = nesterov ? fmaf(momentum, bv, gv) : bv;
+    }
+    const float pn = fmaf(-lr, upd, pv);
+    p[i] = pn;
+    return pn;
+  }
+};
+
+// Adam / AdamW as torch 2.11's `_multi_tensor_adam` (torch/optim/adam.py, capturable=False) computes it on CUDA, one
+// IEEE rounding per ATen kernel (the foreach kernels run in fp32 with their scalars rounded to fp32):
+//   g = g * grad_scale                                  (only when grad_scale != 1)
+//   L2:    g = fma(wd, p, g)                            _foreach_add(grads, params, alpha=wd)
+//   AdamW: p = p * decay                                _foreach_mul_(params, 1 - lr * wd)
+//   m = fma(w, g - m, m)                                _foreach_lerp_(exp_avgs, grads, 1 - beta1)  (ATen Lerp.h,
+//                                                       |w| < 0.5; otherwise g - (g - m) * (1 - w))
+//   v = fma(1 - beta2, g * g, v * beta2)                _foreach_mul_ + _foreach_addcmul_ (DeviceAddCmulCdiv.cuh)
+//   d = sqrt(v) / bc2_sqrt + eps                        _foreach_sqrt, _foreach_div_, _foreach_add_
+//   p = fma(step_size, m / d, p)                        _foreach_addcdiv_(params, exp_avgs, d, step_size)
+// step_size, bc2_sqrt and decay are per tensor (each tensor has its own step count): adam_scalars_kernel writes them
+// before this kernel runs.
+struct AdamRule {
+  struct Args {
+    float* master;
+    const float* grad;
+    float* exp_avg;
+    float* exp_avg_sq;
+    const float4* scalars;  // per tensor: step_size, bc2_sqrt, decay (adam_scalars_kernel)
+    float w1, w1c, beta2, c2, eps, wd, grad_scale;  // fp32 of 1 - beta1, 1 - w1, beta2, 1 - beta2, eps, weight_decay
+    int decoupled;
+  };
+  float* __restrict__ p;
+  const float* __restrict__ g;
+  float* __restrict__ m;
+  float* __restrict__ v;
+  float step_size, bc2_sqrt, decay, w1, w1c, beta2, c2, eps, wd, grad_scale;
+  bool decoupled;
+  __device__ __forceinline__ AdamRule(const Args& a, int t, const b200unet_flat_tensor& D)
+      : p(a.master + D.offset), g(a.grad + D.offset), m(a.exp_avg + D.offset), v(a.exp_avg_sq + D.offset),
+        w1(a.w1), w1c(a.w1c), beta2(a.beta2), c2(a.c2), eps(a.eps), wd(a.wd), grad_scale(a.grad_scale),
+        decoupled(a.decoupled != 0) {
+    const float4 s = a.scalars[t];
+    step_size = s.x;
+    bc2_sqrt = s.y;
+    decay = s.z;
+  }
+  __device__ __forceinline__ float operator()(int i) const {
+    float pv = p[i];
+    float gv = __ldg(g + i);
+    const float mv = m[i], vv = v[i];
+    if (grad_scale != 1.f) gv = __fmul_rn(gv, grad_scale);
+    if (wd != 0.f) {
+      if (decoupled) pv = __fmul_rn(pv, decay);
+      else gv = fmaf(wd, pv, gv);
+    }
+    const float diff = __fsub_rn(gv, mv);
+    const float mn = fabsf(w1) < 0.5f ? fmaf(w1, diff, mv) : fmaf(-diff, w1c, gv);
+    const float gg = __fmul_rn(gv, gv);
+    const float vb = __fmul_rn(vv, beta2);
+    const float vn = c2 == 1.f ? fmaf(gv, gv, vb) : fmaf(c2, gg, vb);  // addcmul with value 1 is a single fma
+    const float d = __fadd_rn(__fdiv_rn(__fsqrt_rn(vn), bc2_sqrt), eps);
+    const float pn = fmaf(step_size, __fdiv_rn(mn, d), pv);
+    m[i] = mn;
+    v[i] = vn;
+    p[i] = pn;
+    return pn;
+  }
+};
+
+template <class Rule>
+__global__ void __launch_bounds__(kFlatThreads) flat_step_kernel(const b200unet_flat_tensor* __restrict__ T, int count,
+                                                                  const __grid_constant__ typename Rule::Args A) {
   int lo = 0, hi = count;
   const int b = blockIdx.x;
   while (hi - lo > 1) {
@@ -84,31 +185,12 @@ __global__ void __launch_bounds__(kFlatThreads) sgd_flat_kernel(const b200unet_f
   }
   const b200unet_flat_tensor D = T[lo];
   if (!(D.flags & 1)) return;
-  const bool first = (D.flags & 2) != 0;
-  float* __restrict__ p = master + D.offset;
-  const float* __restrict__ g = grad + D.offset;
-  float* __restrict__ buf = mom ? mom + D.offset : nullptr;
+  const Rule update(A, lo, D);
   __nv_bfloat16* wf = static_cast<__nv_bfloat16*>(D.wf);
   __nv_bfloat16* wdp = static_cast<__nv_bfloat16*>(D.wd);
   __nv_bfloat16* ws = static_cast<__nv_bfloat16*>(D.ws);
   const int kk = D.ksize * D.ksize;
   const int per_o = D.cin * kk;
-  // the per-element update: torch's CUDA foreach arithmetic, operation by operation
-  auto update = [&](int i) -> float {
-    const float pv = p[i];
-    float gv = g[i];
-    if (grad_scale != 1.f) gv = __fmul_rn(gv, grad_scale);
-    if (wd != 0.f) gv = fmaf(wd, pv, gv);
-    float upd = gv;
-    if (momentum != 0.f) {
-      const float bv = first ? gv : __fadd_rn(__fmul_rn(buf[i], momentum), gv);
-      buf[i] = bv;
-      upd = nesterov ? fmaf(momentum, bv, gv) : bv;
-    }
-    const float pn = fmaf(-lr, upd, pv);
-    p[i] = pn;
-    return pn;
-  };
   if (wf && kk == 9 && (D.cin & 31) == 0 && (D.cout & 31) == 0 && D.cin_pad == D.cin && D.cout_pad == D.cout) {
     // ---- 3x3 conv weights of the tensor-core path: TILES of 32 output x 32 input channels x 9 taps (9216 elements).
     // Walking a tensor in OIHW order made every bf16 pack store a lone 2-byte write (2-3 per parameter, 0.45 ms per
@@ -174,6 +256,55 @@ __global__ void __launch_bounds__(kFlatThreads) sgd_flat_kernel(const b200unet_f
         ws[((static_cast<int64_t>(ph * 2 + pw) * D.cin + ci) * 4 + (dh * 2 + dw)) * D.cout + o] = v;
       }
     }
+  }
+}
+
+// x * y in double-double arithmetic (hi + lo, |lo| <= ulp(hi) / 2)
+__device__ __forceinline__ void dd_mul(double& xh, double& xl, double yh, double yl) {
+  const double p = __dmul_rn(xh, yh);
+  double e = fma(xh, yh, -p);
+  e = fma(xh, yl, fma(xl, yh, e));
+  xh = __dadd_rn(p, e);
+  xl = __dsub_rn(e, __dsub_rn(xh, p));
+}
+
+// beta ** n for an integer n >= 1, correctly rounded to double like the libm pow behind Python's `beta ** step`:
+// binary powering in double-double (relative error ~1e-30), rounded once at the end.  CUDA's pow() is within 2 ulp,
+// which the cancellation in 1 - beta2 ** step (beta2 = 0.999) can carry into the fp32 scalars.
+__device__ double pow_steps(double beta, unsigned n) {
+  double rh = 1.0, rl = 0.0, bh = beta, bl = 0.0;
+  while (true) {
+    if (n & 1u) dd_mul(rh, rl, bh, bl);
+    n >>= 1;
+    if (!n) break;
+    dd_mul(bh, bl, bh, bl);
+  }
+  return rh;
+}
+
+// The host-side half of torch's Adam step, on the device so that a CUDA graph replays it: advance the fp32 step count
+// of every tensor that has a gradient (_foreach_add_(state_steps, 1)) and form its scalars in double exactly as
+// adam.py does -- bc1 = 1 - beta1 ** step, step_size = (lr / bc1) * -1, bc2_sqrt = (1 - beta2 ** step) ** 0.5,
+// decay = 1 - lr * weight_decay -- rounded to fp32 as ATen rounds a scalar list.  One block; the flat step kernel runs
+// after it on the same stream.
+__global__ void __launch_bounds__(128) adam_scalars_kernel(const b200unet_flat_tensor* __restrict__ T, int count,
+                                                           float* __restrict__ steps, float4* __restrict__ scalars,
+                                                           double lr_arg, const double* __restrict__ lr_dev,
+                                                           double beta1, double beta2, double wd) {
+  const double lr = lr_dev ? *lr_dev : lr_arg;
+  for (int t = threadIdx.x; t < count; t += blockDim.x) {
+    if (!(T[t].flags & 1)) continue;
+    const float s = __fadd_rn(steps[t], 1.f);
+    steps[t] = s;
+    const unsigned n = static_cast<unsigned>(s);
+    const double bc1 = __dsub_rn(1.0, pow_steps(beta1, n));
+    const double bc2 = __dsub_rn(1.0, pow_steps(beta2, n));
+    float4 o;
+    o.x = __double2float_rn(-__ddiv_rn(lr, bc1));
+    o.y = __double2float_rn(__dsqrt_rn(bc2));
+    o.z = __double2float_rn(__dsub_rn(1.0, __dmul_rn(lr, wd)));
+    o.w = 0.f;
+    scalars[t] = o;
   }
 }
 
@@ -331,9 +462,30 @@ extern "C" int b200unet_sgd_flat_step(const b200unet_flat_tensor* table_dev, int
                                       void* stream) {
   B200_CHECK_ARG(table_dev && master && grad && count > 0 && total_blocks > 0, "sgd_flat_step: null pointer or empty table");
   B200_CHECK_ARG(momentum == 0.f || momentum_buf, "sgd_flat_step: momentum buffer required");
-  sgd_flat_kernel<<<total_blocks, kFlatThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      table_dev, count, master, grad, momentum_buf, lr, momentum, weight_decay, nesterov, grad_scale, lr_dev);
-  B200_LAUNCH_CHECK("sgd_flat_kernel");
+  const SgdRule::Args a{master, grad, momentum_buf, lr, momentum, weight_decay, grad_scale, nesterov, lr_dev};
+  flat_step_kernel<SgdRule><<<total_blocks, kFlatThreads, 0, static_cast<cudaStream_t>(stream)>>>(table_dev, count, a);
+  B200_LAUNCH_CHECK("flat_step_kernel<SgdRule>");
+  return 0;
+}
+
+extern "C" int b200unet_adam_flat_step(const b200unet_flat_tensor* table_dev, int count, int total_blocks, float* master,
+                                       const float* grad, float* exp_avg, float* exp_avg_sq, float* steps,
+                                       float* scalars_ws, double lr, const double* lr_dev, double beta1, double beta2,
+                                       double eps, double weight_decay, int decoupled, float grad_scale, void* stream) {
+  B200_CHECK_ARG(table_dev && master && grad && exp_avg && exp_avg_sq && steps && scalars_ws && count > 0 &&
+                     total_blocks > 0, "adam_flat_step: null pointer or empty table");
+  B200_CHECK_ARG((reinterpret_cast<uintptr_t>(scalars_ws) & 15) == 0, "adam_flat_step: scalars_ws must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  adam_scalars_kernel<<<1, 128, 0, st>>>(table_dev, count, steps, reinterpret_cast<float4*>(scalars_ws), lr, lr_dev,
+                                          beta1, beta2, weight_decay);
+  B200_LAUNCH_CHECK("adam_scalars_kernel");
+  // the fp32 scalars of the foreach calls, rounded from the double the Python code computes
+  const float w1 = static_cast<float>(1.0 - beta1);
+  const AdamRule::Args a{master, grad, exp_avg, exp_avg_sq, reinterpret_cast<const float4*>(scalars_ws), w1, 1.f - w1,
+                         static_cast<float>(beta2), static_cast<float>(1.0 - beta2), static_cast<float>(eps),
+                         static_cast<float>(weight_decay), grad_scale, decoupled};
+  flat_step_kernel<AdamRule><<<total_blocks, kFlatThreads, 0, st>>>(table_dev, count, a);
+  B200_LAUNCH_CHECK("flat_step_kernel<AdamRule>");
   return 0;
 }
 

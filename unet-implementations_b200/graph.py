@@ -15,8 +15,9 @@ What is captured: every kernel of libb200unet.so on the capture stream, the side
 masks) and the allocations of the step (a private pool: replays reuse the same addresses, which is also why the TMA
 descriptors baked into the kernel parameters stay valid).  The reference has no counterpart (its loop is eager,
 Our_UNet/src/train.py:630-670).  The optimizer step can be part of the graph: `FusedSGD(..., model=model,
-capturable=True)` reads its learning rate from a device scalar, which replay() refreshes from `param_groups` -- what
-LambdaLR changes every epoch (train.py:454-477) -- so the schedule works without re-capturing.
+capturable=True)` and `FusedAdam(..., model=model, capturable=True)` read their learning rate from a device scalar,
+which replay() refreshes from `param_groups` -- what LambdaLR / CosineAnnealingLR change every epoch (train.py:454-477)
+-- so the schedule works without re-capturing.
 """
 from __future__ import annotations
 
@@ -27,7 +28,8 @@ import torch
 
 class GraphedStep:
     """step_fn: zero_grad(set_to_none=True) -> forward -> loss -> backward [-> optimizer.step()], returning the loss.
-    optimizer: a `FusedSGD(..., model=model, capturable=True)` whose step() is INSIDE step_fn -- the whole training step
+    optimizer: a `FusedSGD(..., model=model, capturable=True)` or `FusedAdam(..., model=model, capturable=True)` whose
+    step() is INSIDE step_fn -- the whole training step
     then replays as one graph; its learning rate lives in a device scalar that replay() refreshes from param_groups
     (what LambdaLR updates), so the schedule keeps working without re-capturing."""
 

@@ -16,6 +16,12 @@ Two modes:
   same offsets, and ONE launch (b200unet_sgd_flat_step) scales the gradient, updates master + momentum and EMITS
   the bf16 [Cout,3,3,Cin] / [Cin,3,3,Cout] / stride-2 packs the conv kernels read, which `UNet` then uses directly:
   no repack kernels between the optimizer and the next forward, and packs that cannot go stale.
+
+`FusedAdam(model.parameters(), ..., model=model)` is the autoencoder trainer's `torch.optim.Adam`
+(AE_pretrained/reconstruction/src/train.py:390-394; AdamW with `decoupled_weight_decay=True`) in the same flat form:
+exp_avg / exp_avg_sq at the flat offsets, the per-parameter step counts in device memory, ONE prologue + ONE flat launch
+(b200unet_adam_flat_step) that emits the packs like FusedSGD's.  Bit-identical to torch.optim.Adam on CUDA
+(tests/test_gpu_adam.py), and its state_dict() has torch.optim.Adam's layout, so either optimizer resumes the other.
 """
 from __future__ import annotations
 
@@ -37,6 +43,23 @@ def _bump_versions(params) -> None:
     torch.autograd.graph.increment_version(list(params))
 
 
+def _sync_lr(opt, dtype) -> None:
+    """The device copy of param_groups[0]["lr"] that a capturable flat optimizer's kernel reads (`opt._lr_dev`)."""
+    if not opt.capturable or opt._flat is None:
+        return
+    dev = opt._flat.master.device
+    if opt._lr_dev is None:
+        opt._lr_dev = torch.zeros(1, dtype=dtype, device=dev)
+        opt._lr_host = torch.zeros(1, dtype=dtype).pin_memory()
+        opt._lr_last = None
+    lr = float(opt.param_groups[0]["lr"])
+    if lr != opt._lr_last:
+        torch.cuda.current_stream().synchronize()  # the pinned scalar may still be in flight from the last change
+        opt._lr_host[0] = lr
+        opt._lr_dev.copy_(opt._lr_host, non_blocking=True)
+        opt._lr_last = lr
+
+
 class FusedSGD(torch.optim.Optimizer):
     def __init__(self, params, lr=1e-3, momentum=0.0, dampening=0.0, weight_decay=0.0, nesterov=False, model=None,
                  grad_scale: float = 1.0, capturable: bool = False):
@@ -56,7 +79,7 @@ class FusedSGD(torch.optim.Optimizer):
         if model is not None:
             if len(self.param_groups) != 1:
                 raise ValueError("FusedSGD(model=...): the flat step supports one parameter group (the trainer has one)")
-            self._flat = _FlatState(model, self.param_groups[0]["params"])
+            self._flat = _FlatState(model, self.param_groups[0]["params"], "FusedSGD")
 
     # ------------------------------------------------------------------------------------------------ step
     @torch.no_grad()
@@ -104,19 +127,7 @@ class FusedSGD(torch.optim.Optimizer):
     def sync_lr(self):
         """capturable mode: copy the current learning rate (what LambdaLR wrote into param_groups) to the device scalar
         the captured optimizer kernel reads.  Called by step() when eager, and by GraphedStep.replay() before a replay."""
-        if not self.capturable or self._flat is None:
-            return
-        dev = self._flat.master.device
-        if self._lr_dev is None:
-            self._lr_dev = torch.zeros(1, dtype=torch.float32, device=dev)
-            self._lr_host = torch.zeros(1, dtype=torch.float32).pin_memory()
-            self._lr_last = None
-        lr = float(self.param_groups[0]["lr"])
-        if lr != self._lr_last:
-            torch.cuda.current_stream().synchronize()  # the pinned scalar may still be in flight from the last change
-            self._lr_host[0] = lr
-            self._lr_dev.copy_(self._lr_host, non_blocking=True)
-            self._lr_last = lr
+        _sync_lr(self, torch.float32)
 
     def _flat_step(self):
         group = self.param_groups[0]
@@ -132,7 +143,7 @@ class FusedSGD(torch.optim.Optimizer):
         with torch.cuda.device(fs.master.device):
             _lib.call("b200unet_sgd_flat_step", ctypes.c_void_p(fs.table_dev.data_ptr()), fs.count, fs.total_blocks,
                       ctypes.c_void_p(fs.master.data_ptr()), ctypes.c_void_p(fs.sink.flat.data_ptr()),
-                      ctypes.c_void_p(fs.momentum.data_ptr()) if mom != 0 else None, float(group["lr"]), mom,
+                      ctypes.c_void_p(fs.bufs["momentum_buffer"].data_ptr()) if mom != 0 else None, float(group["lr"]), mom,
                       float(group["weight_decay"]), int(bool(group["nesterov"])), float(self.grad_scale),
                       ctypes.c_void_p(self._lr_dev.data_ptr()) if self._lr_dev is not None else None,
                       ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
@@ -140,11 +151,119 @@ class FusedSGD(torch.optim.Optimizer):
             fs.after_step(self.state, mom != 0)
 
 
-class _FlatState:
-    """Flat master / momentum buffers in the layout of the model's flat gradient sink, the bf16 pack arena and the
-    device descriptor table of b200unet_sgd_flat_step."""
+class FusedAdam(torch.optim.Optimizer):
+    """torch.optim.Adam (AdamW with decoupled_weight_decay=True) as one flat step over the model's buffers.
 
-    def __init__(self, model, params: List[nn.Parameter]):
+    Only the flat form exists: `model=` is required and the parameters become views of one fp32 master buffer, exactly
+    as with FusedSGD(model=...).  Each step is two launches (b200unet_adam_flat_step): a one-block prologue that
+    advances the step counts and forms torch's bias corrections in double, and the flat kernel that updates
+    parameters, exp_avg and exp_avg_sq and emits the bf16 conv weight packs.  The result is bit-identical to
+    torch.optim.Adam (foreach, CUDA) for grad_scale 1, and state_dict() / load_state_dict() interchange with it.
+
+    grad_scale multiplies every gradient inside the step (the 1 / world size of ddp.BucketedGradAllReduce).
+    capturable: the learning rate is read from a float64 device scalar, so that step() can sit inside a CUDA graph
+    (graph.GraphedStep(..., optimizer=opt) refreshes it before each replay); betas, eps and weight_decay are fixed at
+    capture.  Not implemented (ValueError): amsgrad, maximize, differentiable, fused, more than one parameter group.
+    """
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, *,
+                 decoupled_weight_decay: bool = False, model=None, grad_scale: float = 1.0, capturable: bool = False,
+                 amsgrad: bool = False, maximize: bool = False, foreach=None, differentiable: bool = False, fused=None):
+        for name, on in (("amsgrad", amsgrad), ("maximize", maximize), ("differentiable", differentiable),
+                         ("fused", fused)):
+            if on:
+                raise ValueError(f"FusedAdam: {name}=True is not implemented")
+        if model is None:
+            raise ValueError("FusedAdam needs model=...: it steps the model's flat parameter and gradient buffers")
+        if not 0.0 <= float(lr):
+            raise ValueError(f"Invalid learning rate: {lr}")
+        if not 0.0 <= float(eps):
+            raise ValueError(f"Invalid epsilon value: {eps}")
+        if not (0.0 <= float(betas[0]) < 1.0 and 0.0 <= float(betas[1]) < 1.0):
+            raise ValueError(f"Invalid beta parameters: {betas}")
+        if not 0.0 <= float(weight_decay):
+            raise ValueError(f"Invalid weight_decay value: {weight_decay}")
+        # the group has torch.optim.Adam's keys, so that a state_dict of either optimizer loads into the other
+        # ("capturable" is left out: it means device-side step counts and different arithmetic to torch)
+        super().__init__(params, dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, amsgrad=False,
+                                      maximize=False, foreach=foreach, differentiable=False, fused=None,
+                                      decoupled_weight_decay=bool(decoupled_weight_decay)))
+        if len(self.param_groups) != 1:
+            raise ValueError("FusedAdam: the flat step supports one parameter group")
+        self.grad_scale = float(grad_scale)
+        self.capturable = bool(capturable)
+        self._lr_dev: Optional[torch.Tensor] = None
+        self._lr_host: Optional[torch.Tensor] = None
+        self._flat = _FlatState(model, self.param_groups[0]["params"], "FusedAdam", buffers=("exp_avg", "exp_avg_sq"),
+                                step_counters=True)
+        self._scalars = torch.empty(4 * self._flat.count, dtype=torch.float32, device=self._flat.master.device)
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        group = self.param_groups[0]
+        for name in ("amsgrad", "maximize", "differentiable", "fused"):  # a loaded state_dict may ask for them
+            if group.get(name):
+                raise ValueError(f"FusedAdam: {name}=True is not implemented")
+        fs = self._flat
+        capturing = torch.cuda.is_current_stream_capturing()
+        if not capturing:
+            fs.sync(self.state, True)
+            self.sync_lr()
+        elif not self.capturable or self._lr_dev is None or any(f < 0 for f in fs.flags):
+            raise RuntimeError("FusedAdam: capture step() with capturable=True and after one eager step (it creates the "
+                               "optimizer state and uploads the tensor table)")
+        beta1, beta2 = group["betas"]
+        with torch.cuda.device(fs.master.device):
+            _lib.call("b200unet_adam_flat_step", ctypes.c_void_p(fs.table_dev.data_ptr()), fs.count, fs.total_blocks,
+                      ctypes.c_void_p(fs.master.data_ptr()), ctypes.c_void_p(fs.sink.flat.data_ptr()),
+                      ctypes.c_void_p(fs.bufs["exp_avg"].data_ptr()), ctypes.c_void_p(fs.bufs["exp_avg_sq"].data_ptr()),
+                      ctypes.c_void_p(fs.steps.data_ptr()), ctypes.c_void_p(self._scalars.data_ptr()),
+                      float(group["lr"]), ctypes.c_void_p(self._lr_dev.data_ptr()) if self._lr_dev is not None else None,
+                      float(beta1), float(beta2), float(group["eps"]), float(group["weight_decay"]),
+                      int(bool(group["decoupled_weight_decay"])), float(self.grad_scale),
+                      ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
+        if not capturing:
+            fs.after_step(self.state, True)
+        return loss
+
+    def sync_lr(self):
+        """capturable mode: copy the current learning rate (what a scheduler wrote into param_groups) to the float64
+        device scalar the captured prologue reads.  Called by step() when eager, and by GraphedStep.replay()."""
+        _sync_lr(self, torch.float64)
+
+    def state_dict(self):
+        """torch.optim.Adam's layout: per parameter `step` (fp32 scalar tensor on the CPU), `exp_avg`, `exp_avg_sq`.
+        The step counts live on the device and are read back here (one synchronising copy)."""
+        sd = super().state_dict()
+        fs = self._flat
+        host = fs.steps.cpu()
+        where = {v.data_ptr(): i for i, v in enumerate(fs.step_views)}
+        out = {}
+        for k, st in sd["state"].items():
+            st = dict(st)
+            s = st.get("step")
+            if s is not None and s.is_cuda and s.data_ptr() in where:
+                st["step"] = host[where[s.data_ptr()]].clone()
+            out[k] = st
+        sd["state"] = out
+        return sd
+
+
+class _FlatState:
+    """Flat master and optimizer-state buffers in the layout of the model's flat gradient sink, the bf16 pack arena and
+    the device descriptor table of the flat step entry points (b200unet_sgd_flat_step, b200unet_adam_flat_step).
+
+    `buffers` names the per-parameter state tensors the optimizer keeps (torch's names: "momentum_buffer" for SGD,
+    "exp_avg" and "exp_avg_sq" for Adam); each is one flat buffer at the gradient offsets, and `state[p][name]` is a
+    view of it.  `step_counters`: an fp32 step count per parameter in device memory (Adam's state["step"]), also held
+    in `state[p]` as a view."""
+
+    def __init__(self, model, params: List[nn.Parameter], owner: str, buffers=("momentum_buffer",),
+                 step_counters: bool = False):
         sink = sink_of(model)
         if sink is None:
             sink = FlatGradSink(model)
@@ -154,19 +273,27 @@ class _FlatState:
         self.params = [p for p in sink.params if id(p) in wanted]
         missing = wanted - {id(p) for p in self.params}
         if missing:
-            raise ValueError("FusedSGD(model=...): every optimised parameter must be a trainable parameter of the model")
+            raise ValueError(f"{owner}(model=...): every optimised parameter must be a trainable parameter of the model")
         for p in self.params:
             if not (p.is_cuda and p.dtype == torch.float32):
-                raise RuntimeError("FusedSGD(model=...): move the model to its CUDA device first (fp32 parameters)")
+                raise RuntimeError(f"{owner}(model=...): move the model to its CUDA device first (fp32 parameters)")
         dev = sink.flat.device
         self.master = torch.zeros(sink.numel, dtype=torch.float32, device=dev)
-        self.momentum = torch.zeros(sink.numel, dtype=torch.float32, device=dev)
+        self.bufs = {name: torch.zeros(sink.numel, dtype=torch.float32, device=dev) for name in buffers}
         self.mviews: Dict[int, torch.Tensor] = {}
-        self.bviews: Dict[int, torch.Tensor] = {}
+        self.views: Dict[str, Dict[int, torch.Tensor]] = {name: {} for name in buffers}
         for p in self.params:
             off = sink.offsets[id(p)]
             self.mviews[id(p)] = self.master[off:off + p.numel()].view(p.shape)
-            self.bviews[id(p)] = self.momentum[off:off + p.numel()].view(p.shape)
+            for name, buf in self.bufs.items():
+                self.views[name][id(p)] = buf[off:off + p.numel()].view(p.shape)
+        self._fresh: List[nn.Parameter] = []
+        self.steps = torch.zeros(len(self.params), dtype=torch.float32, device=dev) if step_counters else None
+        self.step_views = [self.steps[i] for i in range(len(self.params))] if step_counters else None
+        # (state name, id(p) -> view) in the order torch creates the state entries
+        self._entries = [(name, self.views[name]) for name in buffers]
+        if step_counters:
+            self._entries.insert(0, ("step", {id(p): v for p, v in zip(self.params, self.step_views)}))
         self._adopt_parameters()
         self._build_packs()
         self.block = _lib.call("b200unet_sgd_flat_block_elems")
@@ -250,33 +377,46 @@ class _FlatState:
                 ext[id(w)] = spec
         model._ext_packs = ext
 
-    def sync(self, state, has_momentum: bool):
-        """Host-side bookkeeping before the launch: parameters / momentum buffers re-pointed by someone else are adopted
+    def sync(self, state, stateful: bool):
+        """Host-side bookkeeping before the launch: parameters / state buffers re-pointed by someone else are adopted
         again, gradients that autograd did not leave in the flat buffer are copied there, and the per-tensor flags
         (has a gradient / first momentum step) are uploaded when they changed."""
         self._adopt_parameters()
         sink = self.sink
         changed = False
+        entries = self._entries
+        self._fresh = []  # parameters whose state entries after_step() creates
         for i, p in enumerate(self.params):
             g = p.grad
             flag = 0
             if g is not None:
                 flag = 1
-                gv = sink._views.get(id(p))
+                key = id(p)
+                gv = sink._views.get(key)
                 if gv is None:
                     off = sink.offsets[id(p)]
                     gv = sink._views[id(p)] = sink.flat[off:off + p.numel()].view(p.shape)
                 if g.data_ptr() != gv.data_ptr():
                     gv.copy_(g)  # a cloned / accumulated / externally produced gradient: bring it into the flat buffer
-                if has_momentum:
+                if stateful:
                     st = state[p]
-                    buf = st.get("momentum_buffer")
-                    bv = self.bviews[id(p)]
-                    if buf is None:
-                        flag |= 2
-                    elif buf.data_ptr() != bv.data_ptr():  # loaded by load_state_dict: adopt
-                        bv.copy_(buf)
-                        st["momentum_buffer"] = bv
+                    missing = None
+                    for name, views in entries:  # state loaded by load_state_dict is adopted into the flat buffers
+                        t = st.get(name)
+                        if t is None:
+                            missing = (missing or []) + [name]
+                        else:
+                            v = views[key]
+                            if t.data_ptr() != v.data_ptr():
+                                v.copy_(t)
+                                st[name] = v
+                    if missing:
+                        self._fresh.append(p)
+                        if self.steps is None:
+                            flag |= 2  # SGD: the kernel initialises the momentum buffer with the gradient, as torch does
+                        else:
+                            for name in missing:  # Adam starts from zero moments and step 0
+                                (self.step_views[i] if name == "step" else self.views[name][id(p)]).zero_()
             if flag != self.flags[i]:
                 self.flags[i] = flag
                 self.table_host[i].flags = flag
@@ -288,7 +428,7 @@ class _FlatState:
             # the pinned staging buffer must not be rewritten before this copy has run
             torch.cuda.current_stream().synchronize()
 
-    def after_step(self, state, has_momentum: bool):
+    def after_step(self, state, stateful: bool):
         upd = [p for i, p in enumerate(self.params) if self.flags[i] & 1]
         if not upd:
             return
@@ -297,5 +437,9 @@ class _FlatState:
             spec = self.packs.get(id(p))
             if spec is not None:
                 spec["version"] = p._version  # the packs were emitted from exactly these values
-            if has_momentum and "momentum_buffer" not in state[p]:
-                state[p]["momentum_buffer"] = self.bviews[id(p)]
+        if stateful:
+            for p in self._fresh:  # first step of p: its state entries are views of the flat buffers
+                st = state[p]
+                for name, views in self._entries:
+                    if name not in st:
+                        st[name] = views[id(p)]
