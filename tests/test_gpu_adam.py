@@ -33,6 +33,9 @@ def _unet(kind):
         from unet_implementations_b200.models.autoencoder import Autoencoder
         return Autoencoder(encoder_dropout_rates=[0.0, 0.0, 0.05, 0.1, 0.15, 0.15],
                            decoder_dropout_rates=[0.15, 0.1, 0.1, 0.05, 0.0]).cuda().train()
+    if kind == "gray":  # 1 input channel: the flat step emits a stem pack for the first conv
+        from unet_implementations_b200.models.unet import UNet
+        return UNet(in_channels=1, n_stages=4, features_per_stage=[32, 64, 128, 128]).cuda().train()
     if kind == "clip":
         from unet_implementations_b200.models.clip_unet import UNet as ClipUNet
         return ClipUNet(n_stages=4, features_per_stage=[32, 64, 128, 128], encoder_dropout_rates=[0] * 4,
@@ -44,7 +47,7 @@ def _task(kind, size, b=2, seed=0):
     """(inputs, loss_fn, target) of one model kind: SimpleLoss on segmentation labels, MSELoss on an image."""
     from unet_implementations_b200.models.losses import MSELoss, SimpleLoss
     g = torch.Generator().manual_seed(seed)
-    x = torch.randn(b, 3, size, size, generator=g).cuda()
+    x = torch.randn(b, 1 if kind == "gray" else 3, size, size, generator=g).cuda()
     if kind.startswith("ae"):
         return (x,), MSELoss(), torch.rand(b, 3, size, size, generator=g).cuda()
     t = torch.randint(0, 3, (b, size, size), generator=g)
@@ -109,7 +112,7 @@ WD = {"none": {}, "l2": dict(weight_decay=1e-2), "adamw": dict(weight_decay=1e-2
 
 @pytest.mark.parametrize("kind,size,wd", [("small", 64, "none"), ("small", 64, "l2"), ("small", 64, "adamw"),
                                           ("full", 128, "l2"), ("ae", 64, "none"), ("ae", 64, "adamw"),
-                                          ("ae_full", 128, "none")])
+                                          ("ae_full", 128, "none"), ("gray", 32, "none"), ("gray", 64, "none")])
 def test_fused_adam_is_bit_identical_to_torch_adam(kind, size, wd):
     from unet_implementations_b200.optim import FusedAdam
     ma = _unet(kind)
@@ -346,3 +349,38 @@ def test_capturing_before_the_first_eager_step_is_a_clear_error():
     with pytest.raises(RuntimeError, match="capturable=True and after one eager step"):
         with torch.cuda.graph(graph):
             opt.step()
+
+
+@pytest.mark.parametrize("kind,opt,features,repacks", [("full", "sgd", None, 0), ("ae", "adam", None, 0),
+                                                       ("clip", "adam", "spatial", 0), ("clip", "adam", "pooled", 1)])
+def test_eager_step_runs_no_pack_kernel_with_a_flat_optimizer(kind, opt, features, repacks):
+    """A pack cache whose reuse rule never matched would still train bit for bit, but repack every conv every step:
+    count the pack entry points of the third eager step.  Under constant (pooled) CLIP features the fusion conv runs
+    on its first half of input channels, a pack the emitted full-width one cannot serve, rebuilt once per step."""
+    from unet_implementations_b200 import _lib
+    from unet_implementations_b200.optim import FusedAdam, FusedSGD
+    model = _unet(kind)
+    inputs, loss_fn, target = _task(kind, 64)
+    if features == "pooled":
+        inputs = (inputs[0], inputs[1].mean((2, 3), keepdim=True))
+    if opt == "sgd":
+        o = FusedSGD(model.parameters(), lr=1e-3, momentum=0.9, nesterov=True, model=model)
+    else:
+        o = FusedAdam(model.parameters(), lr=1e-3, model=model)
+
+    def step():
+        o.zero_grad(set_to_none=True)
+        loss_fn(model(*inputs), target).backward()
+        o.step()
+
+    step(), step()
+    prof = _lib.PROFILER = _lib.EventProfiler()
+    try:
+        step()
+    finally:
+        _lib.PROFILER = None
+    torch.cuda.synchronize()
+    calls = {k: len(v) for k, v in prof.pairs.items()}
+    assert calls[f"b200unet_{opt}_flat_step"] == 1 and calls["b200unet_conv_fprop"] > 0
+    assert calls.get("b200unet_pack_conv_weights", 0) == repacks
+    assert calls.get("b200unet_pack_s2_dgrad_weights", 0) == 0

@@ -74,6 +74,26 @@ def test_fused_sgd_with_unet_is_bit_identical_to_torch_sgd(flat, full, size):
         assert torch.equal(sa["state"][k]["momentum_buffer"], sb["state"][k]["momentum_buffer"])
 
 
+@pytest.mark.parametrize("size", [32, 64])
+def test_flat_sgd_with_a_single_channel_unet_is_bit_identical_to_torch_sgd(size):
+    """The flat step emits a stem pack (input channels padded to 32) for a 1-channel first conv.  Images narrower than
+    64 px take the plain first-conv route, which must get its own pack, not the emitted stem pack."""
+    from unet_implementations_b200.models.unet import UNet
+    from unet_implementations_b200.optim import FusedSGD
+    torch.manual_seed(1234)
+    ma = UNet(in_channels=1, n_stages=4, features_per_stage=[32, 64, 128, 128]).cuda().train()
+    mb = copy.deepcopy(ma)
+    x, t = _batch(size)
+    x = x[:, :1].contiguous()
+    kw = dict(lr=0.005, momentum=0.99, nesterov=True, weight_decay=1e-4)
+    ra = _run(ma, torch.optim.SGD(ma.parameters(), **kw), x, t, 2)
+    rb = _run(mb, FusedSGD(mb.parameters(), model=mb, **kw), x, t, 2)
+    for s, ((la, lossa, pa), (lb, lossb, pb)) in enumerate(zip(ra, rb)):
+        assert torch.equal(la, lb), f"step {s}: logits differ by {(la - lb).abs().max().item():.3e}"
+        assert torch.equal(lossa, lossb)
+        assert all(torch.equal(u, v) for u, v in zip(pa, pb))
+
+
 def test_flat_step_emits_the_packs_the_pack_kernels_would():
     from unet_implementations_b200 import ops
     from unet_implementations_b200.optim import FusedSGD

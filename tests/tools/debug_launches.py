@@ -35,5 +35,5 @@ def sgd_step():
 sgd_step(); sgd_step(); sgd_step()
 print("step + FusedSGD(model):", count(sgd_step))
 w = model.encoder_stages[2].block[0].weight
-spec = model._ext_packs[id(w)]
-print("version", w._version, "spec", spec["version"], "ext ok:", model._ext(w, torch.bfloat16) is not None)
+pk = model._packs.emitted[id(w)]
+print("version", w._version, "emitted pack stamped at", pk.version, "current:", pk.valid(w, True))

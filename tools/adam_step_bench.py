@@ -2,7 +2,7 @@
 MSELoss) with the Adam optimizer its trainer uses (AE_pretrained/reconstruction/src/train.py:390-394), four ways:
 
   torch_adam_eager   forward + MSE + backward + torch.optim.Adam(foreach=True).step(), eager; the next forward re-packs
-                     every conv weight Adam changed (UNet._packed*), which is part of the time
+                     every conv weight Adam changed (packs.PackStore), which is part of the time
   fused_adam_eager   the same with FusedAdam(model=...): one prologue + one flat launch, packs emitted by the step
   no_opt_graph       forward + MSE + backward only, replayed as one CUDA graph
   fused_adam_graph   forward + MSE + backward + FusedAdam(capturable=True).step(), replayed as one CUDA graph

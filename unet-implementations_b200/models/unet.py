@@ -26,9 +26,9 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 try:  # package import (unet_implementations_b200.models.unet)
-    from .. import ops
+    from .. import ops, packs
 except ImportError:  # imported as top-level `models.unet` through the drop-in shim directory
-    from unet_implementations_b200 import ops
+    from unet_implementations_b200 import ops, packs
 
 BF16 = torch.bfloat16
 
@@ -217,7 +217,7 @@ class UNet(nn.Module):
         self.skip_constant_features = True
         self.producer_sums_dgrad = os.environ.get("B200UNET_PRODUCER_SUMS_DGRAD", "0") == "1"  # dgrad epilogues (a loss)
         self._side_streams: Dict[int, torch.cuda.Stream] = {}
-        self._pack_cache: Dict[int, Tuple[int, torch.Tensor, Optional[torch.Tensor]]] = {}
+        self._packs = packs.PackStore()  # the conv weight packs the kernels read (packs.py)
         # "bf16": production path (tcgen05 convs, NHWC bf16 arena).  "fp32": verification mode -- the same fused
         # forward/backward with an fp32 arena, the storage-type templates of the norm/resample/head kernels and the
         # direct fp32 convs; agrees with the reference to 1e-4 on loss and every gradient (tests/test_gpu_model.py)
@@ -253,6 +253,11 @@ class UNet(nn.Module):
                 if m.bias is not None:
                     nn.init.constant_(m.bias, 0)
 
+    @property
+    def _ext_packs(self):  # read-only view of _packs.emitted: id(weight) -> {"key", "version", "wf", "wd", "ws"}
+        return {k: dict(key=p.layout.kind, version=p.version, wf=p.wf, wd=p.wd, ws=p.ws)
+                for k, p in self._packs.emitted.items()}
+
     # ------------------------------------------------------------------------------------------------ plan
     def _layers(self):
         """Flat list of fused units in forward order with their role in the graph."""
@@ -268,100 +273,6 @@ class UNet(nn.Module):
             for i, u in enumerate(us):
                 layers.append(dict(kind="dec", stage=j, idx=i, last=(i == len(us) - 1), unit=u))
         return layers
-
-    def _ext(self, w: nn.Parameter, dtype):
-        """The bf16 packs of weight `w` maintained by the fused optimizer step (optim.FusedSGD(model=...) emits them from
-        the updated master weights inside its one launch), if they were made from exactly the current values."""
-        packs = getattr(self, "_ext_packs", None)
-        if not packs or dtype != BF16:
-            return None
-        spec = packs.get(id(w))
-        if spec is None or spec["version"] != w._version or spec["wf"].device != w.device:
-            return None  # someone else wrote the weight since (load_state_dict, an in-place init): repack as usual
-        return spec
-
-    def _packed(self, conv: nn.Conv2d, need_dgrad: bool, dtype=BF16):
-        """Repacks of a conv weight for the conv kernels ([Cout,3,3,Cin] and [Cin,3,3,Cout], bf16 or fp32), cached on
-        the parameter's version counter."""
-        w = conv.weight
-        ext = self._ext(w, dtype)
-        if ext is not None and (ext["wd"] is not None or not need_dgrad):
-            return ext["wf"], ext["wd"]
-        key = id(w)
-        ver = w._version
-        hit = self._pack_cache.get(key)
-        if hit is not None and hit[0] == ver and hit[1].device == w.device and (hit[2] is not None or not need_dgrad) \
-                and hit[3] == w.data_ptr() and hit[1].dtype == dtype:
-            return hit[1], hit[2]
-        wf, wd = ops.pack_conv_weights(w, need_dgrad=need_dgrad, dtype=dtype)
-        self._pack_cache[key] = (ver, wf, wd, w.data_ptr())
-        return wf, wd
-
-    def _packed_stem(self, conv: nn.Conv2d):
-        """bf16 [Cout,3,3,32] pack of the stem weight (input channels zero-padded to 32), cached like _packed."""
-        w = conv.weight
-        ext = self._ext(w, BF16)
-        if ext is not None and ext["key"] == "stem":
-            return ext["wf"]
-        key = ("stem", id(w))
-        hit = self._pack_cache.get(key)
-        if hit is not None and hit[0] == w._version and hit[1].device == w.device and hit[3] == w.data_ptr():
-            return hit[1]
-        wf = ops.pack_stem_weights(w)
-        self._pack_cache[key] = (w._version, wf, None, w.data_ptr())
-        return wf
-
-    def _packed_s2(self, conv: nn.Conv2d, wd: torch.Tensor):
-        """Parity-stacked dgrad pack of a stride-2 conv with Cin in {32, 64} (ops.pack_s2_dgrad_weights), cached on the
-        identity of the ordinary dgrad pack it is derived from; None when the path does not apply."""
-        ext = self._ext(conv.weight, BF16)
-        if ext is not None and ext["wd"] is wd:
-            return ext["ws"]
-        key = ("s2", id(conv.weight))
-        hit = self._pack_cache.get(key)
-        if hit is not None and hit[0] is wd:
-            return hit[1]
-        ws = ops.pack_s2_dgrad_weights(wd)
-        self._pack_cache[key] = (wd, ws, None, None)
-        return ws
-
-    def _packed_1x1(self, conv: nn.Conv2d, need_dgrad: bool, dtype, cin_used: Optional[int] = None):
-        """A 1x1 conv on the 3x3 conv kernels: its weight as the centre tap of a zero 3x3 kernel (the fusion layer is
-        2.4 GFLOP per image this way, 0.6 % of the step), packed and cached like _packed."""
-        w = conv.weight
-        cin = conv.in_channels if cin_used is None else cin_used  # leading input channels only (constant extra features)
-        ext = self._ext(w, dtype)
-        if ext is not None and ext["key"] == "k1" and cin == conv.in_channels:
-            return ext["wf"], ext["wd"]
-        key = ("k1", id(w), cin)
-        hit = self._pack_cache.get(key)
-        if hit is not None and hit[0] == w._version and hit[1].device == w.device and hit[3] == w.data_ptr() \
-                and hit[1].dtype == dtype and (hit[2] is not None or not need_dgrad):
-            return hit[1], hit[2]
-        w3 = torch.zeros((conv.out_channels, cin, 3, 3), dtype=torch.float32, device=w.device)
-        w3[:, :, 1, 1] = w.detach()[:, :cin, 0, 0]
-        wf, wd = ops.pack_conv_weights(w3, need_dgrad=need_dgrad, dtype=dtype)
-        self._pack_cache[key] = (w._version, wf, wd, w.data_ptr())
-        return wf, wd
-
-    def _packed_head(self, conv: nn.Conv2d, need_dgrad: bool, dtype):
-        """Packs of a 3x3 head conv whose OUTPUT channels are zero-padded (32 for the bf16 tensor-core kernels, 8 for
-        the fp32 direct kernels), cached like _packed."""
-        w = conv.weight
-        ext = self._ext(w, dtype)
-        if ext is not None and ext["key"] == "head":
-            return ext["wf"], ext["wd"]
-        key = ("head", id(w))
-        hit = self._pack_cache.get(key)
-        if hit is not None and hit[0] == w._version and hit[1].device == w.device and hit[3] == w.data_ptr() \
-                and hit[1].dtype == dtype and (hit[2] is not None or not need_dgrad):
-            return hit[1], hit[2]
-        cpad = 32 if dtype == BF16 else 8
-        wp = torch.zeros((cpad, conv.in_channels, 3, 3), dtype=torch.float32, device=w.device)
-        wp[:conv.out_channels] = w.detach()
-        wf, wd = ops.pack_conv_weights(wp, need_dgrad=need_dgrad, dtype=dtype)
-        self._pack_cache[key] = (w._version, wf, wd, w.data_ptr())
-        return wf, wd
 
     # normalisation applied to uint8 HWC input batches (the dataset's, train.py:303-308)
     input_mean = (0.485, 0.456, 0.406)
@@ -567,7 +478,7 @@ def _forward_impl(ctx, model: UNet, x: torch.Tensor, params):
                     xin32 = ops.preprocess_u8_nhwc32(x_u8, model.input_mean, model.input_std)
                 else:
                     xin32 = ops.image_to_nhwc32(x)
-                y, stats = ops.conv_fprop(xin32, model._packed_stem(conv), 1, want_stats=True)
+                y, stats = ops.conv_fprop(xin32, model._packs.get(conv, "stem", BF16, False)[0], 1, want_stats=True)
                 rec["stem"] = True
                 rec["xin32"] = xin32 if need_grad else None
             elif cin == 3 and cout == 32 and stride == 1 and adt == BF16:
@@ -575,7 +486,7 @@ def _forward_impl(ctx, model: UNet, x: torch.Tensor, params):
                 rec["stem"] = True
             else:
                 xin = ops.nchw_to_nhwc(_image(), out=_padded_nhwc(B, H, W, cin, dev, adt))
-                wf, wd = model._packed(conv, False, adt)
+                wf, wd = model._packs.get(conv, "conv", adt, False)
                 y, stats = _conv_fwd(xin, wf, stride)
                 rec["xin"] = xin
                 rec["stem"] = False
@@ -584,13 +495,13 @@ def _forward_impl(ctx, model: UNet, x: torch.Tensor, params):
                 if conv.kernel_size != (1, 1) or conv.in_channels != feats[-1] + extra.shape[1]:
                     raise NotImplementedError("b200unet: the fusion layer must be a 1x1 conv over cat([bottleneck, features])")
                 if const_extra:
-                    wf, wd = model._packed_1x1(conv, need_grad, adt, cin_used=feats[-1])
+                    wf, wd = model._packs.get(conv, "k1", adt, need_grad, cin_used=feats[-1])
                     rec["cin_used"] = feats[-1]
                 else:
                     cur = catf
-                    wf, wd = model._packed_1x1(conv, need_grad, adt)
+                    wf, wd = model._packs.get(conv, "k1", adt, need_grad)
             else:
-                wf, wd = model._packed(conv, need_grad, adt)
+                wf, wd = model._packs.get(conv, "conv", adt, need_grad)
             y, stats = _conv_fwd(cur, wf, stride)
             rec["xin"] = cur
             rec["wd"] = wd
@@ -637,7 +548,7 @@ def _forward_impl(ctx, model: UNet, x: torch.Tensor, params):
         # zero-padded (bf16: to the tensor-core kernels' 32; fp32: to the 8-channel vector width), then bias + sigmoid
         if head.out_channels > 4 or head.bias is None or head.in_channels % 32 != 0:
             raise NotImplementedError("b200unet: the reconstruction head is built for Conv2d(32k -> <=4, 3x3, bias) + Sigmoid")
-        wfh, wdh = model._packed_head(head, need_grad, adt)
+        wfh, wdh = model._packs.get(head, "head", adt, need_grad)
         yh, _ = ops.conv_fprop(cur, wfh, 1, want_stats=False, simt=not _use_tc(head.in_channels, wfh.shape[0]))
         logits = ops.recon_head_forward(yh[..., :head.out_channels], head.bias)
         if need_grad:
@@ -864,7 +775,7 @@ def _backward_impl(ctx, dlogits):
         dx = None
         if not last:
             wd = rec["wd"]
-            ws2 = model._packed_s2(conv, wd) if (stride == 2 and not simt and wd.dtype == BF16) else None
+            ws2 = model._packs.s2(conv, wd) if (stride == 2 and not simt and wd.dtype == BF16) else None
             split_out = None
             if (L["kind"] == "dec" and L["idx"] == 0 and not simt and stride == 1 and dy.dtype == BF16
                     and cin == 96 and feats[n - 1 - L["stage"]] == 64 and model.split_concat_grad):
@@ -939,7 +850,7 @@ class _BlockFunction(torch.autograd.Function):
         recs = []
         need_grad = any(ctx.needs_input_grad)
         for conv, norm, act, drop in units:
-            wf, wd = ops.pack_conv_weights(conv.weight, need_dgrad=need_grad)
+            wf, wd = packs.build(conv.weight, packs.layout(conv, "conv"), need_grad)  # no pack store here
             y, stats = _conv_fwd(cur, wf, conv.stride[0])
             scale = None
             if drop is not None and block.training and drop.drop_prob > 0:

@@ -26,15 +26,13 @@ exp_avg / exp_avg_sq at the flat offsets, the per-parameter step counts in devic
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import torch
 import torch.nn as nn
 
 from . import _lib
 from .flat import FlatGradSink, sink_of
-
-BF16 = torch.bfloat16
 
 
 def _bump_versions(params) -> None:
@@ -253,9 +251,31 @@ class FusedAdam(torch.optim.Optimizer):
         return sd
 
 
+def flat_pack_kinds(model) -> List[Tuple[nn.Conv2d, str]]:
+    """(conv, pack kind) of every conv whose bf16 packs the flat step emits: the tensor-core shapes, and the stem whose
+    input channels the tensor-core stem route pads to 32 (packs.py)."""
+    layers = model._layers()
+    out = []
+    for L in layers:
+        conv = L["unit"][0]  # 3x3 (ConvBlock.units)
+        if L is layers[0] and conv.in_channels <= 8 and conv.out_channels == 32 and conv.stride[0] == 1:
+            out.append((conv, "stem"))
+        elif conv.in_channels % 32 == 0 and conv.out_channels % 32 == 0:
+            out.append((conv, "conv"))
+    fusion = model._fusion_unit()
+    if fusion is not None and tuple(fusion[0].kernel_size) == (1, 1) and fusion[0].in_channels % 32 == 0 \
+            and fusion[0].out_channels % 32 == 0:
+        out.append((fusion[0], "k1"))
+    head = model._head_conv()
+    if model.head_kind != "seg1x1" and head.in_channels % 32 == 0 and head.out_channels <= 4:
+        out.append((head, "head"))
+    return out
+
+
 class _FlatState:
-    """Flat master and optimizer-state buffers in the layout of the model's flat gradient sink, the bf16 pack arena and
-    the device descriptor table of the flat step entry points (b200unet_sgd_flat_step, b200unet_adam_flat_step).
+    """Flat master and optimizer-state buffers in the layout of the model's flat gradient sink, the bf16 packs the step
+    emits (packs.PackStore.emit) and the device descriptor table of the flat step entry points (b200unet_sgd_flat_step,
+    b200unet_adam_flat_step).
 
     `buffers` names the per-parameter state tensors the optimizer keeps (torch's names: "momentum_buffer" for SGD,
     "exp_avg" and "exp_avg_sq" for Adam); each is one flat buffer at the gradient offsets, and `state[p][name]` is a
@@ -295,7 +315,9 @@ class _FlatState:
         if step_counters:
             self._entries.insert(0, ("step", {id(p): v for p, v in zip(self.params, self.step_views)}))
         self._adopt_parameters()
-        self._build_packs()
+        mine = {id(p) for p in self.params}
+        emitted = {id(conv.weight): model._packs.emit(conv, kind) for conv, kind in flat_pack_kinds(model)
+                   if id(conv.weight) in mine}
         self.block = _lib.call("b200unet_sgd_flat_block_elems")
         self.count = len(self.params)
         self.flags: List[int] = [-1] * self.count
@@ -307,13 +329,13 @@ class _FlatState:
             t.numel = p.numel()
             t.first_block = blocks
             blocks += (p.numel() + self.block - 1) // self.block
-            spec = self.packs.get(id(p))
-            if spec is not None:
-                t.cout, t.cin, t.ksize = spec["cout"], spec["cin"], spec["ksize"]
-                t.cout_pad, t.cin_pad = spec["cout_pad"], spec["cin_pad"]
-                t.wf = spec["wf"].data_ptr()
-                t.wd = spec["wd"].data_ptr() if spec["wd"] is not None else None
-                t.ws = spec["ws"].data_ptr() if spec["ws"] is not None else None
+            pk = emitted.get(id(p))
+            if pk is not None:
+                lay = pk.layout
+                t.cout, t.cin, t.ksize, t.cout_pad, t.cin_pad = lay.cout, lay.cin, lay.ksize, lay.cout_pad, lay.cin_pad
+                t.wf = pk.wf.data_ptr()
+                t.wd = pk.wd.data_ptr() if pk.wd is not None else None
+                t.ws = pk.ws.data_ptr() if pk.ws is not None else None
         self.total_blocks = blocks
         nbytes = ctypes.sizeof(self.table_host)
         self.table_dev = torch.empty(nbytes, dtype=torch.uint8, device=dev)
@@ -328,54 +350,6 @@ class _FlatState:
                 if p.data_ptr() != v.data_ptr():
                     v.copy_(p.detach())
                     p.data = v
-
-    def _build_packs(self):
-        """bf16 packs for every conv weight the tensor-core path reads, filled once from the current weights with the
-        library's pack kernels and from then on by the optimizer kernel itself; registered with the model."""
-        from . import ops
-        model = self.model
-        self.packs: Dict[int, dict] = {}
-        ext = {}
-        mine = {id(p) for p in self.params}
-        layers = model._layers()
-        fusion = model._fusion_unit() if hasattr(model, "_fusion_unit") else None
-        units = [(L["unit"][0], "conv") for L in layers]
-        if fusion is not None:
-            units.append((fusion[0], "fusion"))
-        head = model._head_conv()
-        if getattr(model, "head_kind", "seg1x1") != "seg1x1":
-            units.append((head, "head3x3"))
-        first_conv = layers[0]["unit"][0]
-        with torch.no_grad():
-            for conv, kind in units:
-                w = conv.weight
-                if id(w) not in mine or id(w) in self.packs:
-                    continue
-                cout, cin = conv.out_channels, conv.in_channels
-                spec = None
-                if kind == "conv" and conv is first_conv and cin <= 8 and cout == 32 and conv.stride[0] == 1:
-                    wf = ops.pack_stem_weights(w)  # [Cout,3,3,32], input channels zero-padded
-                    spec = dict(cout=cout, cin=cin, ksize=3, cout_pad=cout, cin_pad=32, wf=wf, wd=None, ws=None, key="stem")
-                elif kind == "conv" and cin % 32 == 0 and cout % 32 == 0 and tuple(conv.kernel_size) == (3, 3):
-                    wf, wd = ops.pack_conv_weights(w, need_dgrad=True)
-                    ws = ops.pack_s2_dgrad_weights(wd) if conv.stride[0] == 2 else None
-                    spec = dict(cout=cout, cin=cin, ksize=3, cout_pad=cout, cin_pad=cin, wf=wf, wd=wd, ws=ws, key="conv")
-                elif kind == "fusion" and tuple(conv.kernel_size) == (1, 1) and cin % 32 == 0 and cout % 32 == 0:
-                    w3 = torch.zeros((cout, cin, 3, 3), dtype=torch.float32, device=w.device)
-                    w3[:, :, 1, 1] = w.detach()[:, :, 0, 0]
-                    wf, wd = ops.pack_conv_weights(w3, need_dgrad=True)
-                    spec = dict(cout=cout, cin=cin, ksize=1, cout_pad=cout, cin_pad=cin, wf=wf, wd=wd, ws=None, key="k1")
-                elif kind == "head3x3" and cin % 32 == 0 and cout <= 4:
-                    wp = torch.zeros((32, cin, 3, 3), dtype=torch.float32, device=w.device)
-                    wp[:cout] = w.detach()
-                    wf, wd = ops.pack_conv_weights(wp, need_dgrad=True)
-                    spec = dict(cout=cout, cin=cin, ksize=3, cout_pad=32, cin_pad=cin, wf=wf, wd=wd, ws=None, key="head")
-                if spec is None:
-                    continue
-                spec["version"] = w._version
-                self.packs[id(w)] = spec
-                ext[id(w)] = spec
-        model._ext_packs = ext
 
     def sync(self, state, stateful: bool):
         """Host-side bookkeeping before the launch: parameters / state buffers re-pointed by someone else are adopted
@@ -433,10 +407,7 @@ class _FlatState:
         if not upd:
             return
         _bump_versions(upd)
-        for p in upd:
-            spec = self.packs.get(id(p))
-            if spec is not None:
-                spec["version"] = p._version  # the packs were emitted from exactly these values
+        self.model._packs.stamp(upd)
         if stateful:
             for p in self._fresh:  # first step of p: its state entries are views of the flat buffers
                 st = state[p]
